@@ -194,6 +194,34 @@ def synthetic_batch(B, seed, pin=False, image=224):
     return {k: v.pin_memory() for k, v in x.items()} if pin else x
 
 
+DUMP_SAMPLE = 1 << 20        # parameter / gradient values kept by --dump-outputs (4 MB each in float32)
+
+
+def optimizer_state(opt, clone=False):
+    """Parameters, Adam moments and the device {lr, step} scalars: everything a training step reads besides its batch."""
+    state = (opt.flat_params, opt.exp_avg, opt.exp_avg_sq, opt._dyn)
+    return tuple(t.clone() for t in state) if clone else state
+
+
+def dump_outputs(out_dir, model, opt, loss, grad_norm):
+    """What one step computed, as DIR/<name>.npy: the loss and gradient norm the step returns, and the same fixed, seeded
+    sample of the updated parameters and of the gradients it left in the arena (trainable parameters in
+    named_parameters() order, padding between the arena's slots excluded)."""
+    import numpy as np
+    arena = model.grad_arena()
+    named = [n for n, p in model.named_parameters() if p.requires_grad]
+    params = torch.cat([opt.flat_params[arena.offsets[n][0]:arena.offsets[n][0] + arena.offsets[n][1]] for n in named])
+    grads = torch.cat([arena.flat[arena.offsets[n][0]:arena.offsets[n][0] + arena.offsets[n][1]] for n in named])
+    idx = torch.randint(0, params.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+    idx = idx.to(params.device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().reshape(1), "grad_norm": grad_norm.detach().reshape(1),
+              "params_sample": params[idx], "grads_sample": grads[idx]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+    _note("wrote %s to %s" % (", ".join(n + ".npy" for n in arrays), out_dir))
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     from multimae_b200 import _lib as L
@@ -214,6 +242,7 @@ def run_ours(args, rank, world, local_rank):
     scaler = NativeScalerWithGradNormCount(enabled=False).attach_arena(model.grad_arena())
     if world > 1:
         attach_data_parallel(model, scaler)
+    initial_state = optimizer_state(opt, clone=True) if args.dump_outputs else None
     torch.manual_seed(1234 + rank)                         # per-rank data / masks (run_pretraining_multimae.py:300)
     B = args.batch
     host = [synthetic_batch(B, 100 * rank + i, pin=True, image=wl["image"]) for i in range(2)]   # 2 x 106 MB: > L2 together
@@ -325,6 +354,19 @@ def run_ours(args, rank, world, local_rank):
         launches = launches_per_step * args.steps          # a replayed graph re-issues the captured launches
     clocks = sampler.stop() if rank == 0 else None
     final_loss = float(loss)
+    if args.dump_outputs:
+        # The float atomics of the step (split-K weight gradients, embedding gradients) add in a different order from run
+        # to run: rounding-level in one step, but the training steps before the last one compound it.  The dumped step
+        # therefore runs the timed path once more, on the last timed batch, from the seeded initial state.
+        with torch.no_grad():
+            for dst, src in zip(optimizer_state(opt), initial_state):
+                dst.copy_(src)
+        opt.invalidate_mirror()
+        opt.ensure_mirror_fresh()                          # a graph replay does not refresh the bf16 weight twin itself
+        loss, grad_norm = train_step(resident[(args.steps - 1) % 2])
+        barrier()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, model, opt, loss, grad_norm)
 
     if rank == 0:
         _note("leg 1 (HBM-resident inputs): %.3f ms/step" % (ms_total / args.steps))
@@ -657,7 +699,12 @@ def main():
     ap.add_argument("--eager-baseline", type=int, default=1, help="0: skip the torch-eager-on-this-GPU sample of the oracle port")
     ap.add_argument("--e2e-probe", action="store_true", help="extra timed loops that isolate the H2D / loss-read costs")
     ap.add_argument("--gemm-shapes", default=None, help="write a per-shape GEMM time table of one profiled step here")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, run the timed path once more on the last timed batch from the seeded "
+                         "initial state and write what it computed to DIR/<name>.npy (float32; same arguments, same inputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.batch is None:
         args.batch = WORKLOADS[args.workload]["batch"]
     _quiet_stdout()

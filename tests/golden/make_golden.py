@@ -1,6 +1,7 @@
-"""Generate the golden fixtures under tests/golden/ from the LIVE reference (runs only where /root/reference exists).
+"""Generate the golden fixtures under tests/golden/ from the LIVE reference, a checkout of EPFL-VILAB/MultiMAE named by
+the environment variable MULTIMAE_REFERENCE.
 
-    python tests/golden/make_golden.py
+    MULTIMAE_REFERENCE=/path/to/MultiMAE python tests/golden/make_golden.py
 
 The reference (EPFL-VILAB/MultiMAE) has no tests or golden vectors of its own, so these fixtures are what pins the
 oracle (oracle/multimae_oracle.py) and, through it, the CUDA path.  The reference is imported unmodified; the only
@@ -18,6 +19,9 @@ Fixtures (all fp32, CPU, torch.save of plain dicts of tensors):
   losses.pt    : the three criteria over norm_pix / label_smoothing / mask, no mask, all-zero mask: values + prediction gradients
   depth_std.pt : truncated depth standardisation; the reference has it inline in train_one_epoch
                  (run_pretraining_multimae.py:487-492), so the statements are cut out of the reference source and executed
+  dropin_schema.json : what the reference script's get_model (run_pretraining_multimae.py:243-290) builds for
+                 pretrain_multimae_base with rgb+depth+semseg (+norm_rgb): state_dict keys and shapes in order, trainable
+                 parameter names, no_weight_decay(), trainable parameter count
 
     python tests/golden/make_golden.py [fixture.pt ...]     (no names: regenerate everything)
 """
@@ -29,13 +33,13 @@ from functools import partial
 
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("MULTIMAE_REFERENCE", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def import_reference():
     if not os.path.isdir(REF):
-        raise SystemExit("reference tree %s not present: fixtures can only be regenerated in the authoring container" % REF)
+        raise SystemExit("set MULTIMAE_REFERENCE to a checkout of EPFL-VILAB/MultiMAE to regenerate the fixtures")
     six = types.ModuleType("torch._six")
     six.inf = math.inf
     sys.modules.setdefault("torch._six", six)
@@ -217,6 +221,28 @@ def record_losses(R, name):
     print("wrote", name, {k: round(float(v["loss_masked"]), 6) for k, v in out["cases"].items()})
 
 
+def record_dropin_schema(name):
+    """The model the reference script's own get_model builds from the arguments of a default pre-training run."""
+    import json
+    sys.path.insert(0, REF)
+    import run_pretraining_multimae as script          # noqa: E402
+    args = types.SimpleNamespace(model="pretrain_multimae_base", in_domains=["rgb", "depth", "semseg"],
+                                 out_domains=["rgb", "depth", "semseg"], patch_size=16, decoder_dim=256, decoder_depth=2,
+                                 decoder_num_heads=8, decoder_use_task_queries=True, decoder_use_xattn=True,
+                                 extra_norm_pix_loss=True, num_global_tokens=1, drop_path=0.0)
+    model = script.get_model(args)
+    out = {"args": vars(args),
+           "state_dict": [[k, list(v.shape)] for k, v in model.state_dict().items()],
+           "trainable": sorted(n for n, p_ in model.named_parameters() if p_.requires_grad),
+           "no_weight_decay": sorted(model.no_weight_decay()),
+           "trainable_numel": sum(p_.numel() for p_ in model.parameters() if p_.requires_grad)}
+    with open(os.path.join(HERE, name), "w") as fh:              # one entry per line
+        fh.write("{\n" + ",\n".join("%s: %s" % (json.dumps(k), json.dumps(v) if k != "state_dict" else
+                                                 "[\n" + ",\n".join(json.dumps(e) for e in v) + "\n]")
+                                     for k, v in out.items()) + "\n}\n")
+    print("wrote", name, "(%d state_dict entries)" % len(out["state_dict"]))
+
+
 def record_depth_standardize(name):
     """Executes the reference's OWN statements (the body of `if standardize_depth and 'depth' in tasks_dict:` in
     train_one_epoch, run_pretraining_multimae.py:487-492) on synthetic depth maps and records input and result."""
@@ -247,8 +273,12 @@ if __name__ == "__main__":
     only = set(sys.argv[1:])
     if only == {"depth_std.pt"}:
         if not os.path.isdir(REF):
-            raise SystemExit("reference tree %s not present" % REF)
+            raise SystemExit("set MULTIMAE_REFERENCE to a checkout of EPFL-VILAB/MultiMAE")
         record_depth_standardize("depth_std.pt")
+        raise SystemExit(0)
+    if only == {"dropin_schema.json"}:
+        import_reference()
+        record_dropin_schema("dropin_schema.json")
         raise SystemExit(0)
     R = import_reference()
     # mask-token queries (multimae/output_adapters.py:214-221): a task that is reconstructed without being fed
@@ -287,6 +317,7 @@ if __name__ == "__main__":
     record_losses(R, "losses.pt")
     record_fixed_masks(R, "fixed_masks.pt")
     record_depth_standardize("depth_std.pt")
+    record_dropin_schema("dropin_schema.json")
     record_sampler(R, "sampler_small.pt", B=16, tokens_per_task=[16, 16, 16], num_encoded=12, alphas=1.0, seed=3)
     record_sampler(R, "sampler_cfg2.pt", B=8, tokens_per_task=[196, 196, 196], num_encoded=98, alphas=1.0, seed=4)
     record_sampler(R, "sampler_alpha.pt", B=8, tokens_per_task=[196, 196], num_encoded=98, alphas=[0.5, 2.0], seed=5)

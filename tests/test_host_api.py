@@ -5,6 +5,8 @@
  * the product path refuses to run without CUDA (no CPU fallback)."""
 import os
 import re
+import subprocess
+import sys
 
 import pytest
 import torch
@@ -47,7 +49,10 @@ def test_abi_exports_every_declared_symbol():
     for name in declared:
         assert getattr(handle, name) is not None
     assert handle.mmae_abi_version() == L.ABI_VERSION
-    assert handle.mmae_launch_count() == 0     # nothing launched on a CPU box
+    # loading the library launches nothing; counted in a fresh process, since GPU tests of this session add to the counter
+    res = subprocess.run([sys.executable, "-c", "import sys; sys.path.insert(0, %r); from multimae_b200 import _lib as L; "
+                          "print(L.lib().mmae_launch_count())" % ROOT], capture_output=True, text=True, timeout=300)
+    assert res.returncode == 0 and res.stdout.split() == ["0"], res.stdout[-500:] + res.stderr[-2000:]
 
 
 def test_state_dict_schema_and_roundtrip(golden_dir):
